@@ -13,7 +13,7 @@ GOLDEN_DIR = os.path.join(ROOT, 'tests', 'golden')
 GOLDEN_CASES = sorted(
     os.path.splitext(os.path.basename(p))[0]
     for p in glob.glob(os.path.join(GOLDEN_DIR, '*.npz'))
-    if not os.path.basename(p).startswith(('cg_', 'big_', 'pbc_', 'ecstr_'))  # iterative-solver / large-molecule fixtures have their own tests
+    if not os.path.basename(p).startswith(('cg_', 'big_', 'pbc_', 'ecstr_', 'dropin_'))  # iterative-solver / large-molecule / CLI fixtures have their own tests
 )
 
 

@@ -11,6 +11,7 @@ GPU box):
     PYTHONPATH=baseline/_ref:. python tests/golden/make_golden.py c60
     PYTHONPATH=baseline/_ref:. python tests/golden/make_golden.py n100
     PYTHONPATH=baseline/_ref:. python tests/golden/make_golden.py pbc_ecstr
+    PYTHONPATH=baseline/_ref:. python tests/golden/make_golden.py dropin
 
 Each fixture holds the inputs (geometries, labels, perms, sig, lam, query geometries) and
 the reference outputs of every hot-path stage: tril_perms_lin (Desc.perm / train.py:897-904),
@@ -316,8 +317,88 @@ def main_n100():
     print('big_n100_m2_s12: K_cols', K_cols.shape, 'size %.0f KB' % (os.path.getsize(out) / 1024))
 
 
+def main_dropin():
+    """The reference's own command line (cli.py: create -> train -> test) on the synthetic dataset of
+    tools/reference_cli_dropin.py, without the engine.  Stores the task the CLI created, the layout of the model
+    file it wrote (keys, shapes, dtypes), c and std, the reference predictor's E / F from that file on the last 8
+    dataset geometries and on every point outside the training and validation sets, and the parameter lists of
+    the reference's GDMLTrain / GDMLPredict that the drop-in must reproduce."""
+    import inspect
+    import json
+    import tempfile
+
+    from sgdml import cli
+    from sgdml.utils import io
+
+    _tspec = importlib.util.spec_from_file_location('dropin', os.path.join(ROOT, 'tools', 'reference_cli_dropin.py'))
+    dropin = importlib.util.module_from_spec(_tspec)
+    _tspec.loader.exec_module(dropin)
+
+    N, n_train, n_valid, n_test, sig = 9, 40, 20, 30, 20
+    with tempfile.TemporaryDirectory() as wd:
+        ds_path = os.path.join(wd, 'dataset.npz')
+        dropin.make_dataset(ds_path, N, n_train + n_valid + n_test + 10)
+        _, dataset = io.is_file_type(ds_path, 'dataset')
+        np.random.seed(0)
+        task_dir = os.path.join(wd, 'tasks')
+        cli.create((ds_path, dataset), None, n_train, n_valid, [sig], False, True, False, True, task_dir=task_dir, command='create')
+        task_files = sorted(f for f in os.listdir(task_dir) if f.startswith('task'))
+        cli.train((task_dir, task_files), (ds_path, dataset), False, True, None, 1, False, command='train')
+        model_files = sorted(f for f in os.listdir(task_dir) if f.startswith('model'))
+        cli.test((task_dir, model_files), (ds_path, dataset), n_test, True, None, 1, False, command='test')
+        with np.load(os.path.join(task_dir, task_files[0]), allow_pickle=True) as f:
+            task = {k: f[k] for k in f.files}
+        with np.load(os.path.join(task_dir, model_files[0]), allow_pickle=True) as f:
+            model = {k: f[k] for k in f.files}
+
+    predictor = GDMLPredict(model, max_processes=1, use_torch=False)
+    n_data = dataset['R'].shape[0]
+    R_query = dataset['R'][-8:].reshape(8, -1)
+    E_q, F_q = predictor.predict(R_query)
+    idxs_out = np.setdiff1d(np.arange(n_data), np.concatenate([task['idxs_train'], task['idxs_valid']]))
+    R_out = dataset['R'][idxs_out].reshape(len(idxs_out), -1)
+    E_out, F_out = predictor.predict(R_out)
+
+    from sgdml.train import GDMLTrain as RefTrain
+
+    sig_of = lambda f: list(inspect.signature(f).parameters)  # noqa: E731
+    signatures = {
+        'GDMLTrain.__init__': sig_of(RefTrain.__init__),
+        'GDMLTrain.train': sig_of(RefTrain.train),
+        'GDMLPredict.__init__': sig_of(GDMLPredict.__init__),
+        'GDMLPredict.predict': sig_of(GDMLPredict.predict),
+    }
+    layout = {
+        'keys': sorted(model.keys()),
+        'shapes': {k: list(np.asarray(model[k]).shape) for k in ('R_desc', 'R_d_desc_alpha', 'alphas_F', 'perms', 'tril_perms_lin')},
+        'dtypes': {k: str(np.asarray(model[k]).dtype) for k in ('R_desc', 'R_d_desc_alpha', 'alphas_F', 'perms', 'tril_perms_lin', 'sig', 'c', 'std')},
+        'solver_name': str(model['solver_name']),
+    }
+    out = os.path.join(HERE, 'dropin_n9_m40.npz')
+    np.savez_compressed(
+        out,
+        reference_version=sgdml.__version__,
+        signatures=json.dumps(signatures),
+        model_layout=json.dumps(layout),
+        **{'task_' + k: v for k, v in task.items()},
+        c=model['c'],
+        std=model['std'],
+        R_query=R_query,
+        E_query=E_q,
+        F_query=F_q,
+        R_out=R_out,
+        F_out_label=dataset['F'][idxs_out].reshape(len(idxs_out), -1),
+        E_out=E_out,
+        F_out=F_out,
+    )
+    print('dropin_n9_m40: %d training points, %d outside points, size %.0f KB' % (len(task['idxs_train']), len(idxs_out),
+                                                                               os.path.getsize(out) / 1024))
+
+
 if __name__ == '__main__':
-    if len(sys.argv) > 1 and sys.argv[1] == 'n100':
+    if len(sys.argv) > 1 and sys.argv[1] == 'dropin':
+        main_dropin()  # separate process: the CLI's own GDMLTrain instances (train.py:336-342)
+    elif len(sys.argv) > 1 and sys.argv[1] == 'n100':
         main_n100()
     elif len(sys.argv) > 1 and sys.argv[1] == 'c60':
         main_c60()

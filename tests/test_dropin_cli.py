@@ -1,74 +1,103 @@
 """(f)1 -- the engine as a drop-in behind the reference's own CLI (north_star; INTEGRATION.md section 4).
-The reference package is the unmodified copy under baseline/_ref (it travels to the GPU box; /root/reference does
-not).  The CLI functions call os._exit on errors, so every flow runs in a subprocess (tools/reference_cli_dropin.py)."""
+The reference's side is frozen in tests/golden/dropin_n9_m40.npz (make_golden.py dropin): the task its CLI created
+(`sgdml create`), the layout of the model file its `sgdml train` / `sgdml test` wrote, the predictions of that model
+by its own GDMLPredict, and the parameter lists of its GDMLTrain / GDMLPredict."""
 
 import inspect
 import json
-import os
-import subprocess
 import sys
+import types
 
 import numpy as np
 import pytest
 
-from conftest import ROOT, rel_err
-
-REF_DIR = os.path.join(ROOT, 'baseline', '_ref')
-needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF_DIR, 'sgdml', 'cli.py')), reason='baseline/_ref not installed')
+from conftest import load_golden, rel_err
 
 
-def _run_tool(engine, workdir):
-    env = dict(os.environ)
-    env['OMP_NUM_THREADS'] = '4'
-    res = subprocess.run(
-        [sys.executable, os.path.join(ROOT, 'tools', 'reference_cli_dropin.py'), '--engine', engine, '--workdir', str(workdir)],
-        env=env, capture_output=True, text=True, timeout=600,
-    )
-    for ln in res.stdout.splitlines():
-        if ln.startswith('DROPIN_JSON '):
-            return json.loads(ln[len('DROPIN_JSON '):])
-    raise AssertionError('no result from the CLI flow (rc %d):\n%s\n%s' % (res.returncode, res.stdout[-2000:], res.stderr[-2000:]))
+@pytest.fixture(scope='module')
+def dropin():
+    g = load_golden('dropin_n9_m40')
+    g['signatures'] = json.loads(str(g['signatures']))
+    g['model_layout'] = json.loads(str(g['model_layout']))
+    return g
 
 
-@needs_ref
-def test_install_rebinds_reference_cli_and_signatures_match():
+def _stand_in_reference(monkeypatch):
+    """A package laid out like the reference (sgdml.cli, sgdml.train) with the host-side task functions the
+    installed training class borrows."""
+
+    class RefTrain(object):
+        def create_task(self, *a, **k):
+            pass
+
+        def create_task_from_model(self, *a, **k):
+            pass
+
+        def draw_strat_sample(self, *a, **k):
+            pass
+
+    pkg = types.ModuleType('sgdml_stand_in')
+    pkg.__path__ = []
+    pkg.cli = types.ModuleType('sgdml_stand_in.cli')
+    pkg.train = types.ModuleType('sgdml_stand_in.train')
+    pkg.cli.GDMLTrain, pkg.cli.GDMLPredict = RefTrain, object
+    pkg.train.GDMLTrain = RefTrain
+    for mod in (pkg, pkg.cli, pkg.train):
+        monkeypatch.setitem(sys.modules, mod.__name__, mod)
+    return pkg, RefTrain
+
+
+def test_install_rebinds_reference_cli_and_signatures_match(monkeypatch, dropin):
     """CPU: the two names the reference CLI instantiates are rebound; constructor / train / predict signatures of
     the engine classes equal the reference's (train.py:306, 836-841; predict.py:249-258, 1146)."""
-    code = (
-        'import sys, json, inspect\n'
-        'sys.path.insert(0, %r); sys.path.insert(0, %r)\n'
-        'import sgdml, sgdml.cli, sgdml.train, sgdml.predict\n'
-        'RefT, RefP = sgdml.train.GDMLTrain, sgdml.predict.GDMLPredict\n'
-        'from sgdml_b200.integration import install_into_reference\n'
-        'T, P = install_into_reference(sgdml)\n'
-        'sig = lambda f: list(inspect.signature(f).parameters)\n'
-        'out = dict(bound=sgdml.cli.GDMLTrain is T and sgdml.cli.GDMLPredict is P,\n'
-        '           init_t=[sig(T.__init__), sig(RefT.__init__)], train=[sig(T.train), sig(RefT.train)],\n'
-        '           init_p=[sig(P.__init__), sig(RefP.__init__)], predict=[sig(P.predict)[:3], sig(RefP.predict)[:3]],\n'
-        '           borrowed=T.create_task is RefT.create_task and T.draw_strat_sample is RefT.draw_strat_sample)\n'
-        'print(json.dumps(out))\n'
-    ) % (ROOT, REF_DIR)
-    res = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, timeout=300)
-    assert res.returncode == 0, res.stderr[-2000:]
-    out = json.loads(res.stdout.strip().splitlines()[-1])
-    assert out['bound'] and out['borrowed']
-    for k in ('init_t', 'train', 'init_p', 'predict'):
-        assert out[k][0] == out[k][1], (k, out[k])
+    from sgdml_b200.integration import install_into_reference
+
+    pkg, RefTrain = _stand_in_reference(monkeypatch)
+    T, P = install_into_reference(pkg)
+    assert pkg.cli.GDMLTrain is T and pkg.cli.GDMLPredict is P
+    assert T.create_task is RefTrain.create_task and T.draw_strat_sample is RefTrain.draw_strat_sample
+    assert T.create_task_from_model is RefTrain.create_task_from_model
+
+    sig = lambda f: list(inspect.signature(f).parameters)  # noqa: E731
+    ref = dropin['signatures']
+    assert sig(T.__init__) == ref['GDMLTrain.__init__']
+    assert sig(T.train) == ref['GDMLTrain.train']
+    assert sig(P.__init__) == ref['GDMLPredict.__init__']
+    assert sig(P.predict)[:3] == ref['GDMLPredict.predict'][:3]
 
 
-@needs_ref
 @pytest.mark.gpu
-def test_reference_cli_train_and_test_through_engine(tmp_path):
-    """`sgdml create` -> `sgdml train` -> `sgdml test` (the reference's own functions) with the engine installed:
-    the .npz it writes has the reference's keys / shapes / dtypes, loads in the UNMODIFIED reference GDMLPredict,
-    and predicts what the reference-trained model predicts (1e-6 rel, north_star)."""
-    eng = _run_tool('b200', tmp_path / 'b200')
-    ref = _run_tool('reference', tmp_path / 'ref')
-    assert eng['model_file'] == ref['model_file']
-    assert eng['keys'] == ref['keys'] and eng['shapes'] == ref['shapes'] and eng['dtypes'] == ref['dtypes']
-    assert eng['solver_name'] == ref['solver_name'] == 'analytic' and eng['n_test'] == ref['n_test']
-    assert rel_err(eng['E_ref_predict'], ref['E_ref_predict']) < 1e-6
-    assert rel_err(eng['F_ref_predict_first'], ref['F_ref_predict_first']) < 1e-6
-    assert abs(eng['c'] - ref['c']) < 1e-6 * abs(ref['c']) and abs(eng['std'] - ref['std']) < 1e-12 * ref['std']
-    # test errors recorded in the model file by cli.test (cli.py:1502-1570) agree to solver accuracy
-    assert abs(eng['f_err']['rmse'] - ref['f_err']['rmse']) < 1e-6 + 0.05 * ref['f_err']['rmse']
+def test_reference_cli_train_and_test_through_engine(tmp_path, dropin):
+    """The task the reference's `sgdml create` wrote, trained by the engine: the model file has the keys / shapes /
+    dtypes of the one the reference's `sgdml train` wrote, read back by a CPU predictor it predicts what the
+    reference-trained model predicts (1e-6 rel, north_star), and its force error on the points outside the training
+    and validation sets agrees with the reference model's."""
+    import sgdml_b200
+    from oracle import predict as opredict
+
+    g = dropin
+    task = {k[len('task_'):]: g[k] for k in g if k.startswith('task_')}
+    model = sgdml_b200.GDMLTrain().train(task)
+    path = tmp_path / 'model.npz'
+    np.savez_compressed(path, **model)  # as cli.py:1098 writes it
+    with np.load(path, allow_pickle=True) as f:
+        model = {k: f[k] for k in f.files}
+
+    ref = g['model_layout']
+    assert sorted(model.keys()) == ref['keys']
+    assert {k: list(np.asarray(model[k]).shape) for k in ref['shapes']} == ref['shapes']
+    assert {k: str(np.asarray(model[k]).dtype) for k in ref['dtypes']} == ref['dtypes']
+    assert str(model['solver_name']) == ref['solver_name'] == 'analytic'
+    c, std = float(model['c']), float(model['std'])
+    assert abs(c - float(g['c'])) < 1e-6 * abs(float(g['c'])) and abs(std - float(g['std'])) < 1e-12 * float(g['std'])
+
+    E, F = opredict.Predictor(model).predict(g['R_query'])
+    assert rel_err(E, g['E_query']) < 1e-6
+    assert rel_err(F, g['F_query']) < 1e-6
+
+    # force error on the held-out points, as `sgdml test` records it (cli.py:1502-1570), through the engine predictor
+    _, F_out = sgdml_b200.GDMLPredict(model).predict(g['R_out'])
+    assert rel_err(F_out, g['F_out']) < 1e-6
+    rmse = np.sqrt(np.mean((F_out - g['F_out_label']) ** 2))
+    rmse_ref = np.sqrt(np.mean((g['F_out'] - g['F_out_label']) ** 2))
+    assert abs(rmse - rmse_ref) < 1e-6 + 0.05 * rmse_ref
