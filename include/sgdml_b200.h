@@ -96,6 +96,15 @@ int sgdml_b200_model_destroy(sgdml_b200_model* model);
 int sgdml_b200_predict(sgdml_b200_model* model, const double* R, int64_t n_geo, double* E,
                        double* F, void* stream);
 
+/* Analytic Hessian (an extension: the reference predicts energies and forces only).  R (B, 3N) ->
+ * H (B, 3N, 3N) = d^2 E / dR^2, row-major, full and symmetric, in model units (energy / length^2), plus E (B,) and
+ * F (B, 3N) as sgdml_b200_predict gives them (E and F may be NULL).  Lattices and alphas_E are honoured.  Every
+ * contraction of this call runs in FP64, whatever sgdml_b200_model_set_contraction_slices chose.  Host or device
+ * pointers; the call synchronises `stream` before it returns.  Molecules up to ~225 atoms (as the predictor);
+ * beyond that SGDML_B200_ERR_UNSUPPORTED.  Derivation: DESIGN.md, "Hessian". */
+int sgdml_b200_predict_hessian(sgdml_b200_model* model, const double* R, int64_t n_geo, double* E, double* F,
+                               double* H, void* stream);
+
 /* Periodic model (predict.py:332-334: lat_and_inv from model['lattice']): query descriptors of
  * sgdml_b200_predict are built with the minimum-image convention.  Both NULL: back to a free molecule. */
 int sgdml_b200_model_set_lattice(sgdml_b200_model* model, const double* lattice, const double* lattice_inv);
@@ -293,7 +302,8 @@ int sgdml_b200_ozaki_debug(int64_t m, int64_t n, int64_t k, const double* A, int
 /* ---------------------------------------------------------------- launch accounting / profiling
  * Kernel families: 0 predictor main kernel, 1 predictor auxiliary kernels, 2 K assembly,
  * 3 DMMA GEMM (Cholesky trailing update), 4 potf2 diagonal tiles, 5 panel TRSM strips,
- * 6 triangular solves, 7 descriptor kernels, 8 misc.
+ * 6 triangular solves, 7 descriptor kernels, 8 misc, 9 the Gram kernel of the analytic Hessian (its other
+ * kernels count as 1, its weight GEMMs as 3).
  * `launches` counts kernel launches per family since the last reset (always on).  With
  * profiling enabled, the library brackets each family's launches with CUDA events on the
  * launching stream and accumulates the device time (this synchronises; benchmarks enable it

@@ -36,6 +36,7 @@ SIGNATURES = {
     ),
     'sgdml_b200_model_destroy': (C.c_int, [c_void_p]),
     'sgdml_b200_predict': (C.c_int, [c_void_p, c_void_p, i64, c_void_p, c_void_p, c_void_p]),
+    'sgdml_b200_predict_hessian': (C.c_int, [c_void_p, c_void_p, i64, c_void_p, c_void_p, c_void_p, c_void_p]),
     'sgdml_b200_model_set_R_d_desc': (C.c_int, [c_void_p, c_void_p]),
     'sgdml_b200_model_set_alphas': (C.c_int, [c_void_p, c_void_p, c_void_p]),
     'sgdml_b200_predict_train': (C.c_int, [c_void_p, i64, i64, C.c_int, c_void_p, c_void_p, c_void_p]),
@@ -194,7 +195,7 @@ def require_gpu():
         raise EngineError('sgdml_b200: no CUDA device visible; this engine has no CPU fallback')
 
 
-KERNEL_FAMILIES = ['predict_main', 'predict_aux', 'assemble', 'gemm', 'potf2', 'trsm', 'trsv', 'desc', 'misc']
+KERNEL_FAMILIES = ['predict_main', 'predict_aux', 'assemble', 'gemm', 'potf2', 'trsm', 'trsv', 'desc', 'misc', 'hessian']
 
 
 def profile_snapshot():

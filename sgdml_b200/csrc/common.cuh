@@ -99,7 +99,8 @@ int num_sms();
 // ------------------------------------------------------------------ launch accounting / profiling
 // Kernel families (ids of sgdml_b200_profile_get).
 enum KernelId { KID_PREDICT_MAIN = 0, KID_PREDICT_AUX = 1, KID_ASSEMBLE = 2, KID_GEMM = 3, KID_POTF2 = 4,
-                KID_TRSM = 5, KID_TRSV = 6, KID_DESC = 7, KID_MISC = 8, KID_COUNT = 9 };
+                KID_TRSM = 5, KID_TRSV = 6, KID_DESC = 7, KID_MISC = 8, KID_HESSIAN = 9,
+                KID_COUNT = 10 };
 void count_launch(int kid, int n = 1);
 // When profiling is enabled, ProfScope records CUDA events around a launch sequence on `s`
 // and adds the elapsed device time to the family's total (synchronises at scope exit).

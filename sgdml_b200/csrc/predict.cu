@@ -25,6 +25,7 @@
 
 #include "common.cuh"
 #include "desc.cuh"
+#include "hessian.cuh"
 #include "solve.cuh"
 
 namespace sgdml {
@@ -1489,8 +1490,11 @@ int64_t chunk_geos(const sgdml_b200_model* m) {
 // Runs the predictor on n_geo queries whose descriptors (xq, gq) are on the device.
 constexpr int64_t GRAPH_MAX_GEO = 16;  // batches up to this size with host buffers replay a captured graph
 // xq == nullptr: the query rows (w.Qg, w.qq) are already in place (k_desc_query_rows)
+// n_splits_out (optional): number of per-split G / Erow planes left in the workspace (stride: rows rounded up to BQ);
+// fp64: the large-descriptor contractions in FP64 DMMA even when the model uses int8 slices
 int run_queries(sgdml_b200_model* m, int slot, const double* xq, const double* gq, int64_t n_geo, double std,
-                double c, double* E_dev, double* F_dev, cudaStream_t s) {
+                double c, double* E_dev, double* F_dev, cudaStream_t s, int* n_splits_out = nullptr,
+                bool fp64 = false) {
   sgdml_b200_model::WS& w = m->ws[slot];
   const int64_t n_rows = n_geo * m->S;
   const int64_t n_rows_pad = (n_rows + m->BQ - 1) / m->BQ * m->BQ;
@@ -1519,7 +1523,7 @@ int run_queries(sgdml_b200_model* m, int slot, const double* xq, const double* g
     // slices of the model matrices are kept with the model, those of Q, C1, C2 are cut per batch; everything is
     // stream-ordered (this path runs once per CG iteration inside sgdml_b200_pcg).  Slice count: m->oz_s
     // (tools/ozaki_study.py predict: forces 8.8e-9 / 6.5e-11 / 5.4e-13 vs FP64 for 4 / 5 / 6 slices).
-    if (m->oz_s >= 2) {
+    if (m->oz_s >= 2 && !fp64) {
       const int S = m->oz_s;
       SG_TRY(ozaki_split(w.Qg, n_rows, m->DS, m->DS, S, w.ozQ.units, w.ozQ.exps, &w.ozQ, s));
       SG_TRY(ozaki_gemm(w.ozQ, m->ozXc, n_rows, m->Mpad, 1.0, 1, w.S1, m->Mpad, S, s));
@@ -1630,6 +1634,7 @@ int run_queries(sgdml_b200_model* m, int slot, const double* xq, const double* g
     SG_CUDA(cudaGetLastError());
     count_launch(KID_PREDICT_AUX);
   }
+  if (n_splits_out != nullptr) *n_splits_out = n_splits;
   return 0;
 }
 
@@ -1979,6 +1984,87 @@ int sgdml_b200_predict(sgdml_b200_model* m, const double* R, int64_t n_geo, doub
     }
   }
   if (host_io) SG_CUDA(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// Analytic Hessian (csrc/hessian.cu).  Per chunk of queries: descriptors, the predictor's run_queries (E, F and the
+// descriptor-space force rows G), then the Hessian kernels on the query rows it leaves in the workspace.
+int sgdml_b200_predict_hessian(sgdml_b200_model* m, const double* R, int64_t n_geo, double* E, double* F, double* H,
+                               void* stream) {
+  SG_TRY(require_device());
+  SG_ARG(m != nullptr && R != nullptr && H != nullptr && n_geo >= 0);
+  if (n_geo == 0) return 0;
+  if ((size_t)m->D * 8 > 200 * 1024) {  // the limit of the predictor's finishing kernel
+    set_last_error("sgdml_b200_predict_hessian: molecule too large (n_atoms <= ~225 supported)");
+    return SGDML_B200_ERR_UNSUPPORTED;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool R_dev = is_device_ptr(R), H_dev = is_device_ptr(H);
+  const bool F_dev = F != nullptr && is_device_ptr(F), E_dev = E != nullptr && is_device_ptr(E);
+  const int dimi = 3 * m->N;
+  const int64_t hsz = (int64_t)dimi * dimi;
+  HessModel hm;
+  hm.N = m->N;
+  hm.D = m->D;
+  hm.DS = m->DS;
+  hm.M = m->M;
+  hm.S = m->S;
+  hm.Mpad = m->Mpad;
+  hm.sig = m->sig;
+  hm.std = m->std;
+  hm.X = m->X;
+  hm.Xc = m->Xc;
+  hm.JA = m->JA;
+  hm.mm = m->mm;
+  hm.xja = m->xja;
+  hm.ae = m->use_ae ? m->ae : nullptr;
+  hm.perm = m->perm;
+  const int64_t chunk = std::min<int64_t>(n_geo, std::min<int64_t>(chunk_geos(m), hessian_chunk_geos(hm)));
+  SG_TRY(ensure_ws(m, 0, chunk));
+  sgdml_b200_model::WS& w = m->ws[0];
+  // one device block for the Hessian workspace (+ the output staging of host H), back to the cache at the end
+  const int64_t last = n_geo - (n_geo - 1) / chunk * chunk;
+  const size_t ws_bytes = std::max(hessian_workspace_bytes(hm, chunk), hessian_workspace_bytes(hm, last));
+  const size_t stage_bytes = H_dev ? 0 : (size_t)chunk * hsz * 8;
+  char* hws = nullptr;
+  SG_CUDA(cached_malloc(&hws, ws_bytes + stage_bytes));
+  auto body = [&]() -> int {
+    for (int64_t g0 = 0; g0 < n_geo; g0 += chunk) {
+      const int64_t ng = std::min<int64_t>(chunk, n_geo - g0);
+      const double* Rd = R + g0 * dimi;
+      if (!R_dev) {
+        SG_CUDA(cudaMemcpyAsync(w.R, Rd, sizeof(double) * ng * dimi, cudaMemcpyHostToDevice, s));
+        Rd = w.R;
+      }
+      SG_TRY(launch_desc_from_R(Rd, ng, m->N, w.xq, w.gq, s, &m->lat));
+      double* Fd = F_dev ? F + g0 * dimi : w.F;
+      double* Ed = (E == nullptr) ? nullptr : (E_dev ? E + g0 : w.E);
+      int n_splits = 1;
+      SG_TRY(run_queries(m, 0, w.xq, w.gq, ng, m->std, m->c, Ed, Fd, s, &n_splits, true));
+      HessChunk hc;
+      hc.ng = ng;
+      hc.xq = w.xq;
+      hc.gq = w.gq;
+      hc.Qg = w.Qg;
+      hc.qq = w.qq;
+      hc.G = w.G;
+      hc.DP = m->DP;
+      hc.n_splits_G = n_splits;
+      hc.plane_rows = (ng * m->S + m->BQ - 1) / m->BQ * m->BQ;
+      hc.H = H_dev ? H + g0 * hsz : reinterpret_cast<double*>(hws + ws_bytes);
+      SG_TRY(run_hessian(hm, hc, hws, s));
+      if (F != nullptr && !F_dev)
+        SG_CUDA(cudaMemcpyAsync(F + g0 * dimi, Fd, sizeof(double) * ng * dimi, cudaMemcpyDeviceToHost, s));
+      if (E != nullptr && !E_dev) SG_CUDA(cudaMemcpyAsync(E + g0, Ed, sizeof(double) * ng, cudaMemcpyDeviceToHost, s));
+      if (!H_dev) SG_CUDA(cudaMemcpyAsync(H + g0 * hsz, hc.H, sizeof(double) * ng * hsz, cudaMemcpyDeviceToHost, s));
+    }
+    return 0;
+  };
+  const int rc = body();
+  cudaError_t e = cudaStreamSynchronize(s);  // the workspace block goes back to the cache: nothing may still use it
+  cached_free(hws);
+  if (rc != 0) return rc;
+  SG_CUDA(e);
   return 0;
 }
 

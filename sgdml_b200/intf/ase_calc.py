@@ -45,6 +45,13 @@ class SGDMLCalculatorCore(object):
         f = f * self.F_to_eV_Ang
         return {'energy': e, 'forces': f.reshape(-1, 3)}
 
+    def compute_hessian(self, positions):
+        """positions (N, 3) in Angstrom -> analytic Hessian d^2 E / dR^2, (3N, 3N) in eV/Ang^2 (the model's
+        Hessian times E_to_eV * Ang_to_R^2).  Rows and columns run over (atom, x/y/z)."""
+        r = np.array(positions, dtype=np.float64) * self.Ang_to_R
+        _, _, h = self.gdml_predict.predict_hessian(r.ravel())
+        return h[0] * (self.E_to_eV * self.Ang_to_R**2)
+
 
 try:
     from ase.calculators.calculator import Calculator
@@ -60,6 +67,17 @@ try:
         def calculate(self, atoms=None, *args, **kwargs):
             super(SGDMLCalculator, self).calculate(atoms, *args, **kwargs)
             self.results = self.compute(atoms.get_positions())
+
+        def get_hessian(self, atoms=None):
+            """Analytic Hessian (3N, 3N) in eV/Ang^2 at the positions of `atoms` (default: the attached atoms).
+            'hessian' is not a standard ASE property, so it is not cached in ``results``.  Harmonic analysis::
+
+                from ase.vibrations import VibrationsData
+                vib = VibrationsData.from_2d(atoms, calc.get_hessian(atoms))
+                vib.get_frequencies()
+            """
+            atoms = atoms if atoms is not None else self.atoms
+            return self.compute_hessian(atoms.get_positions())
 
 except ImportError:
 

@@ -240,29 +240,73 @@ class GDMLPredict(object):
         )
         return (E, F) if return_E else (F,)
 
+    def predict_hessian(self, R, out=None):
+        """Extension: analytic Hessian.  R (B, 3N) [or (3N,)] float64 -> (E (B,), F (B, 3N), H (B, 3N, 3N)), with
+        H = d^2 E / dR^2 full and symmetric in model units (energy / length^2); E and F as ``predict`` gives them.
+        Lattices and alphas_E are honoured.  NumPy in -> NumPy out; torch tensor in (CUDA, or pinned/pageable host)
+        -> torch tensors out on the same device.  `out=(E, F, H)`: preallocated outputs, checked as in ``predict``.
+        All contractions run in FP64, whatever ``set_contraction_slices`` chose."""
+        dim_i = 3 * self.n_atoms
+        if isinstance(R, np.ndarray) or not hasattr(R, 'data_ptr'):
+            R = np.ascontiguousarray(R, dtype=np.float64)
+            if R.ndim == 1:
+                R = R[None, :]
+            if R.size % dim_i != 0 or (R.ndim == 2 and R.shape[1] != dim_i):
+                raise ValueError('R must have 3*n_atoms columns')
+            R = R.reshape(-1, dim_i)
+            n = R.shape[0]
+            alloc = lambda shape: np.empty(shape)  # noqa: E731
+        else:
+            import torch
+
+            if R.dtype != torch.float64:
+                raise ValueError('torch inputs must be float64')
+            R = R.contiguous().reshape(-1, dim_i) if R.dim() != 1 else R.contiguous().reshape(1, dim_i)
+            n = R.shape[0]
+            pin = (not R.is_cuda) and R.is_pinned()  # pinned host tensor in -> pinned host tensors out
+            alloc = lambda shape: torch.empty(shape, dtype=torch.float64, device=R.device, pin_memory=pin)  # noqa: E731
+        if out is None:
+            E, F, H = alloc((n,)), alloc((n, dim_i)), alloc((n, dim_i, dim_i))
+        else:
+            if len(out) != 3 or out[2] is None:
+                raise ValueError('out must be (E, F, H) with H given (E, F may be None)')
+            E, F, H = out
+            self._check_out(R, E, F, n, dim_i)
+            self._check_buf(R, H, (n, dim_i, dim_i), 'H')
+        _lib.check(
+            _lib.lib().sgdml_b200_predict_hessian(
+                self._handle, _lib.ptr(R), n, _lib.ptr(E), _lib.ptr(F), _lib.ptr(H), _lib.current_stream()
+            ),
+            'predict_hessian',
+        )
+        return E, F, H
+
     @staticmethod
     def _check_out(R, E, F, n, dim_i):
         """Output buffers go to the engine as raw double*: wrong dtype / layout / device would corrupt memory."""
         for buf, shape, name in ((F, (n, dim_i), 'F'), (E, (n,), 'E')):
-            if buf is None:
-                continue
-            if tuple(buf.shape) != shape:
-                raise ValueError('out buffer %s has the wrong shape %s (expected %s)' % (name, tuple(buf.shape), shape))
-            if isinstance(buf, np.ndarray):
-                if buf.dtype != np.float64 or not buf.flags['C_CONTIGUOUS'] or not buf.flags['WRITEABLE']:
-                    raise ValueError('out buffer %s must be a writeable C-contiguous float64 array' % name)
-                if not isinstance(R, np.ndarray) and R.is_cuda:
-                    raise ValueError('out buffer %s is a host array but R is a CUDA tensor' % name)
-            else:
-                import torch
+            if buf is not None:
+                GDMLPredict._check_buf(R, buf, shape, name)
 
-                if buf.dtype != torch.float64 or not buf.is_contiguous():
-                    raise ValueError('out buffer %s must be a contiguous float64 tensor' % name)
-                r_dev = None if isinstance(R, np.ndarray) else R.device
-                if buf.is_cuda and (r_dev is None or buf.device != r_dev):
-                    raise ValueError('out buffer %s lives on %s but R does not' % (name, buf.device))
-                if (not buf.is_cuda) and r_dev is not None and r_dev.type == 'cuda':
-                    raise ValueError('out buffer %s is a host tensor but R is a CUDA tensor' % name)
+    @staticmethod
+    def _check_buf(R, buf, shape, name):
+        if tuple(buf.shape) != shape:
+            raise ValueError('out buffer %s has the wrong shape %s (expected %s)' % (name, tuple(buf.shape), shape))
+        if isinstance(buf, np.ndarray):
+            if buf.dtype != np.float64 or not buf.flags['C_CONTIGUOUS'] or not buf.flags['WRITEABLE']:
+                raise ValueError('out buffer %s must be a writeable C-contiguous float64 array' % name)
+            if not isinstance(R, np.ndarray) and R.is_cuda:
+                raise ValueError('out buffer %s is a host array but R is a CUDA tensor' % name)
+        else:
+            import torch
+
+            if buf.dtype != torch.float64 or not buf.is_contiguous():
+                raise ValueError('out buffer %s must be a contiguous float64 tensor' % name)
+            r_dev = None if isinstance(R, np.ndarray) else R.device
+            if buf.is_cuda and (r_dev is None or buf.device != r_dev):
+                raise ValueError('out buffer %s lives on %s but R does not' % (name, buf.device))
+            if (not buf.is_cuda) and r_dev is not None and r_dev.type == 'cuda':
+                raise ValueError('out buffer %s is a host tensor but R is a CUDA tensor' % name)
 
     def kmatvec_train(self, m_begin=0, m_end=None, out=None):
         """Raw (std = 1, c = 0) force sums on training points [m_begin, m_end): the K.v operator
